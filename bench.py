@@ -2,14 +2,16 @@
 """bench.py — PointFusion frames/sec (640x480, B=8 sequences of L=32 frames per GPU, odom='gt', fwd only).
 
     python bench.py [--gpus N --steps K --warmup W]            our CUDA arm
+    python bench.py ... --dump-outputs DIR                     also write the last timed step's result to DIR/*.npy
     python bench.py --impl reference [...]                     the CPU oracle port timed on the host cores
     torchrun ... bench.py --gpus N ...                         one rank per GPU (weak scaling: B=8 per GPU)
 
 One "step" = one whole `PointFusion(odom='gt')(frames)` call over a (B, L) batch of synthetic RGB-D
 sequences = B*L frame updates (per frame: K1r frame records, K2/K3 project+select, K3c per-tile append counts,
-K4 merge+append).  The timed region is EXACTLY --steps steps; because 20 steps are only ~0.1 s, the region is
-measured `--repeats` times back to back (default: enough repeats for >= 100 timed steps) and the MEDIAN region
-is reported (all of them are listed under "timed_regions_ms").
+K4 merge+append).  The timed region is EXACTLY --steps steps; with `--repeats R` it is measured R times back to back
+(default 1) and the MEDIAN region is reported (all of them are listed under "timed_regions_ms").  The inputs are
+seeded, so the same arguments give the same inputs on every run; --dump-outputs writes what the timed path returned
+in its last step, so that two builds can be compared output for output.
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what each key means.
 """
 import argparse
@@ -39,7 +41,9 @@ def parse():
     ap.add_argument("--height", type=int, default=480)
     ap.add_argument("--width", type=int, default=640)
     ap.add_argument("--cpu-sample-frames", type=int, default=12, help="frames of the CPU-baseline sample (B=1)")
-    ap.add_argument("--repeats", type=int, default=0, help="timed regions of --steps steps each (0: ceil(100/steps))")
+    ap.add_argument("--repeats", type=int, default=1, help="timed regions of --steps steps each")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's poses, map sizes and a fixed sample of map rows as DIR/*.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the B=1 / L=32 (config 2) line")
     ap.add_argument("--no-icp", action="store_true", help="skip the secondary ICP-odometry measurement")
@@ -198,6 +202,28 @@ def workload_config(args, world):
     }
 
 
+DUMP_BYTES = 48 << 20  # budget of the sampled map rows in --dump-outputs
+
+
+def dump_outputs(out_dir, pc, poses):
+    """Writes one PointFusion result as float32 / float64 .npy files: the recovered poses, the map sizes and the map's
+    points, normals, colours and confidence counts at a fixed, seeded sample of row indices (map_rows.npy; rows past an
+    element's size are zero).  The whole map (~140 MB at the default workload) is sampled to stay within DUMP_BYTES."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    B, n = pc.points_padded.shape[:2]
+    keep = min(n, DUMP_BYTES // (max(B, 1) * 10 * 4))
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    idx = rows.to(pc.points_padded.device)
+    arrays = {"poses": poses, "num_points": pc.num_points_per_pointcloud.double(), "map_rows": rows.double(),
+              "points": pc.points_padded[:, idx], "normals": pc.normals_padded[:, idx],
+              "colors": pc.colors_padded[:, idx], "features": pc.features_padded[:, idx]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------------
 def main():
     args = parse()
@@ -307,7 +333,8 @@ def main():
         if d2h:
             res = read_back(*prev)
             torch.cuda.current_stream(dev).wait_stream(dl_stream)
-        return res
+            return res
+        return prev[:2]  # (map, poses) of the last step, on the device
 
     def timed(frames, steps, d2h):
         barrier()
@@ -332,15 +359,18 @@ def main():
             all_ms.append(ms)
         return sorted(all_ms)[len(all_ms) // 2], all_ms, res
 
-    repeats = args.repeats if args.repeats > 0 else max(1, -(-100 // max(1, args.steps)))
+    repeats = max(1, args.repeats)
     if world > 1:  # setup, not warm-up: let the caching allocator reach its steady state (two map stores and two sets
         run_steps(frames_dev, 3, d2h=False)  # of gather buffers are alive at once in the pipelined loop)
     run_steps(frames_dev, max(args.warmup, 3), d2h=False)  # same (pipelined) code path as the timed region
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_dev, all_dev, _ = timed_median(frames_dev, args.steps, False, repeats)
+    ms_dev, all_dev, last = timed_median(frames_dev, args.steps, False, repeats)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
     if args.no_e2e:
         ms_e2e, all_e2e = float("nan"), []
     else:

@@ -6,15 +6,17 @@ Imports the reference from /root/reference through tests/golden/ref_loader.py (f
 there) and writes
 
   tests/golden/msrd_b2s3.npz   the reference's own test data and golden vectors (tests/data/msrd_b2s3/*.npy: colors,
-                               depths, intrinsics, poses -> vertex / normal / global maps), re-packed losslessly; the
-                               inputs of the reference's hot-path tests (tests/common.py load_test_data), which
-                               tests/test_gpu_reference_twins.py restates against this package on the GPU
+                               depths, intrinsics, poses -> vertex / normal / global maps); the inputs of the
+                               reference's hot-path tests (tests/common.py load_test_data), which
+                               tests/test_gpu_reference_twins.py restates against this package on the GPU, are kept
+                               losslessly, the four golden maps as every 17th pixel plus checksums (frozen.py)
   tests/golden/ref_slam.npz    reference outputs on seeded synthetic sequences (gradslam_b200.synthetic, the
                                bench's own input distribution: 2 % random depth holes): PointFusion / ICPSLAM
                                final maps + poses for odom in {gt, icp, gradicp}, the frame maps (K1) of one
                                sequence, the three correspondence tables of one fusion step, an ICP / gradICP
                                transform recovery case, and one FULL-SIZE run (640x480, B=1, L=6, odom=gt):
                                per-frame map sizes, float64 checksums and every 53rd surfel of the final map.
+                               Final maps are stored as every 8th surfel plus float64 checksums (frozen.py).
 
 The inputs of ref_slam.npz are NOT stored: the tests regenerate them from the recorded seeds.
 """
@@ -31,6 +33,7 @@ sys.path.insert(0, HERE)
 sys.path.insert(0, ROOT)
 warnings.simplefilter("ignore")
 
+from frozen import PIXEL_STRIDE, narrow_int, pack_rows  # noqa: E402
 from ref_loader import REFERENCE_ROOT, load_reference  # noqa: E402
 
 load_reference()
@@ -61,11 +64,11 @@ FULL_STRIDE = 53   # every 53rd surfel of its final map is stored
 def pack_map(prefix, pc, out):
     out[prefix + "/counts"] = np.array([int(c) for c in pc.num_points_per_pointcloud], dtype=np.int64)
     for b in range(len(pc)):
-        out["%s/points/%d" % (prefix, b)] = pc.points_list[b].numpy()
-        out["%s/normals/%d" % (prefix, b)] = pc.normals_list[b].numpy()
-        out["%s/colors/%d" % (prefix, b)] = pc.colors_list[b].numpy()
+        pack_rows(out, "%s/points/%d" % (prefix, b), pc.points_list[b].numpy())
+        pack_rows(out, "%s/normals/%d" % (prefix, b), pc.normals_list[b].numpy())
+        pack_rows(out, "%s/colors/%d" % (prefix, b), pc.colors_list[b].numpy())
         if pc.has_features:
-            out["%s/ccounts/%d" % (prefix, b)] = pc.features_list[b].numpy()
+            pack_rows(out, "%s/ccounts/%d" % (prefix, b), pc.features_list[b].numpy())
 
 
 def main():
@@ -74,6 +77,8 @@ def main():
     msrd = {k: np.load(os.path.join(d, k + ".npy")) for k in
             ("colors", "depths", "intrinsics", "poses", "vertex_map", "normal_map", "global_vertex_map",
              "global_normal_map")}
+    for k in ("vertex_map", "normal_map", "global_vertex_map", "global_normal_map"):
+        pack_rows(msrd, k, msrd.pop(k).reshape(-1, 3), PIXEL_STRIDE)
     np.savez_compressed(os.path.join(HERE, "msrd_b2s3.npz"), **msrd)
 
     out = {}
@@ -124,11 +129,11 @@ def main():
     t_active = ref_fu.find_active_map_points(pc, live)
     t_similar, mask = ref_fu.find_similar_map_points(pc, live, t_active, slam.dist_th, slam.dot_th)
     t_unique = ref_fu.find_best_unique_correspondences(pc, live, t_similar)
-    out["tables/active"] = t_active.numpy()
-    out["tables/similar"] = t_similar.numpy()
+    out["tables/active"] = narrow_int(t_active.numpy())
+    out["tables/similar"] = narrow_int(t_similar.numpy())
     out["tables/similar_mask"] = mask.numpy()
-    out["tables/unique"] = t_unique.numpy()
-    pack_map("tables/map_before", pc, out)
+    out["tables/unique"] = narrow_int(t_unique.numpy())
+    out["tables/map_before/counts"] = np.array([int(c) for c in pc.num_points_per_pointcloud], dtype=np.int64)
     fused = ref_fu.fuse_with_map(pc.clone(), live, t_unique, slam.sigma, inplace=False)
     pack_map("tables/map_after", fused, out)
     print("tables", t_active.shape, t_similar.shape, t_unique.shape)

@@ -6,7 +6,8 @@ Same mechanism as make_golden.py (reference imported from /root/reference throug
 the default-parameter fixtures leave untouched: distance / angle thresholds and sigma of the fusion, the ICP
 down-sampling ratio, damping, distance threshold and the gradLM gate parameters, a non-square image, a sequence
 whose first pose is not the identity, and five edge cases (all-invalid frames, an empty sequence, partial frames, a
-frame without any correspondence).  Inputs are NOT stored: the tests regenerate them from the recorded seeds.
+frame without any correspondence).  Inputs are NOT stored: the tests regenerate them from the recorded seeds.  Maps are
+stored as every 8th surfel plus float64 checksums (frozen.py).
 """
 import os
 import sys
@@ -29,6 +30,7 @@ from gradslam.structures.rgbdimages import RGBDImages  # noqa: E402
 
 from gradslam_b200.synthetic import make_sequence  # noqa: E402
 from edge_cases import EDGE_CASES, edge_inputs  # noqa: E402
+from frozen import pack_rows  # noqa: E402
 from make_golden import pack_map  # noqa: E402
 
 # (name, class, B, L, H, W, seed, make_sequence kwargs, slam kwargs)
@@ -52,8 +54,8 @@ def main():
         out[name + "/counts"] = np.array([int(c) for c in pc.num_points_per_pointcloud], dtype=np.int64)
         for b in range(len(pc)):
             if out[name + "/counts"][b] > 0:
-                out["%s/points/%d" % (name, b)] = pc.points_list[b].numpy()
-                out["%s/ccounts/%d" % (name, b)] = pc.features_list[b].numpy()
+                pack_rows(out, "%s/points/%d" % (name, b), pc.points_list[b].numpy())
+                pack_rows(out, "%s/ccounts/%d" % (name, b), pc.features_list[b].numpy())
         print(name, out[name + "/counts"])
     for name, cls, B, L, H, W, seed, seq_kw, kw in PARAM_CASES:
         rgb, depth, K, poses = make_sequence(B, L, H, W, seed=seed, **seq_kw)

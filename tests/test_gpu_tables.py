@@ -1,18 +1,16 @@
 """GPU parity for the table-returning association API (index work: bit-exact against the oracle and against the
 tables frozen from the unmodified reference), plus the reference's hand-built known-answer cases."""
 import math
-import os
 
-import numpy as np
 import pytest
 import torch
 
 import gsx_oracle as oracle
+from frozen import load  # tests/golden is on sys.path, see conftest.py
 from gradslam_b200.synthetic import make_sequence
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 DOT_TH = math.cos(20 * math.pi / 180)
 
 
@@ -47,7 +45,7 @@ def test_tables_match_oracle_and_frozen_reference():
     assert torch.equal(unique.cpu(), r_unique)
     assert torch.equal(fu.find_correspondences(pc, live, 0.05, DOT_TH).cpu(), r_unique)
     # the same tables, frozen from the unmodified reference
-    ref = np.load(os.path.join(GOLD, "ref_slam.npz"))
+    ref = load("ref_slam.npz")
     assert torch.equal(active.cpu(), torch.from_numpy(ref["tables/active"]))
     assert torch.equal(similar.cpu(), torch.from_numpy(ref["tables/similar"]))
     assert torch.equal(unique.cpu(), torch.from_numpy(ref["tables/unique"]))

@@ -2,18 +2,15 @@
 outputs frozen from the unmodified reference (tests/golden/ref_slam_params.npz, made by
 tests/golden/make_golden_params.py).  Ground-truth-odometry cases are index / IEEE work end to end and must match the
 oracle bit for bit; ICP cases are held to north_star's tolerances (1e-4 on poses, 1e-3 on fused points)."""
-import os
-
-import numpy as np
 import pytest
 import torch
 
 import gsx_oracle as oracle
+from frozen import assert_rows_close, load  # tests/golden is on sys.path, see conftest.py
 from gradslam_b200.synthetic import make_sequence
 
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 # (name, class, mode, B, L, H, W, seed, make_sequence kwargs, slam kwargs) - the cases of make_golden_params.py
 PARAM_CASES = [
@@ -33,7 +30,7 @@ PARAM_CASES = [
 
 @pytest.fixture(scope="module")
 def frozen():
-    return dict(np.load(os.path.join(GOLD, "ref_slam_params.npz")))
+    return load("ref_slam_params.npz")
 
 
 def _nn_dist(a, b):
@@ -62,10 +59,8 @@ def test_slam_with_other_parameters(frozen, case):
         # ... and within the golden-test tolerances of the frozen reference outputs
         assert got == frozen[name + "/counts"].tolist()
         for b in range(B):
-            torch.testing.assert_close(pc.points_list[b].cpu(), torch.from_numpy(frozen["%s/points/%d" % (name, b)]),
-                                       rtol=0, atol=2e-5)
-            torch.testing.assert_close(pc.features_list[b].cpu(), torch.from_numpy(frozen["%s/ccounts/%d" % (name, b)]),
-                                       rtol=1e-6, atol=1e-7)
+            assert_rows_close(pc.points_list[b], frozen, "%s/points/%d" % (name, b), rtol=0, atol=2e-5)
+            assert_rows_close(pc.features_list[b], frozen, "%s/ccounts/%d" % (name, b), rtol=1e-6, atol=1e-7)
         return
     # ICP odometry: north_star tolerances, against the oracle and against the frozen reference poses
     torch.testing.assert_close(rec.cpu(), ref.poses, rtol=0, atol=1e-4)
@@ -110,5 +105,4 @@ def test_edge_cases(frozen, name):
             assert torch.equal(pc.colors_list[b].cpu(), ref.map.colors[b])
             assert torch.equal(pc.features_list[b].cpu(), ref.map.ccounts[b])
             if n:
-                torch.testing.assert_close(pc.points_list[b].cpu(), torch.from_numpy(frozen["%s/points/%d" % (name, b)]),
-                                           rtol=0, atol=2e-5)
+                assert_rows_close(pc.points_list[b], frozen, "%s/points/%d" % (name, b), rtol=0, atol=2e-5)
