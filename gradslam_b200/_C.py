@@ -68,8 +68,6 @@ SIGNATURES = {
     "gsx_icp_tgt_scratch_bytes": (c_i64, [c_int, c_i64]),
     "gsx_knn1": (c_int, [c_vp, c_vp, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_int, c_vp]),
     "gsx_icp_normal_eq_scratch_bytes": (c_i64, [c_int]),
-    "gsx_icp_normal_eq_fwd": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gsx_icp_normal_eq_bwd": (c_int, [c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "gsx_icp_normal_eq_batched_fwd": (c_int, [c_vp, c_vp, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gsx_icp_normal_eq_batched_bwd": (c_int, [c_vp, c_vp, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
                                               c_vp]),
@@ -79,11 +77,9 @@ SIGNATURES = {
                                    c_vp, c_vp, c_vp, c_vp]),
     "gsx_icp_update_bwd": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_float, c_float, c_float, c_float,
                                    c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
-    "gsx_rigid_transform_fwd": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp]),
     "gsx_rigid_transform_bwd_scratch_bytes": (c_i64, [c_i64]),
     "gsx_rigid_transform_batched_fwd": (c_int, [c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_vp]),
     "gsx_rigid_transform_batched_bwd": (c_int, [c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
-    "gsx_rigid_transform_bwd": (c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "gsx_icp_align_scratch_bytes": (c_i64, [c_int, c_int, c_int]),
     "gsx_icp_align": (
         c_int, [c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_float, c_int, c_float,

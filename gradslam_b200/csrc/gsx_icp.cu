@@ -1168,34 +1168,3 @@ extern "C" int gsx_icp_normal_eq_batched_bwd(const float *src_points, const int3
   GSX_CHECK_LAUNCH("gsx_icp_normal_eq_batched_bwd");
   return 0;
 }
-
-extern "C" int gsx_icp_normal_eq_fwd(const float *src_points, int ns, const float *tgt_points,
-                                     const float *tgt_normals, const int64_t *nn_idx, float *sums_out, void *scratch,
-                                     int64_t scratch_bytes, void *stream) {
-  GSX_CHECK_ARG(src_points && tgt_points && tgt_normals && nn_idx && sums_out && scratch,
-                "gsx_icp_normal_eq_fwd: null pointer");
-  GSX_CHECK_ARG(ns >= 1 && scratch_bytes >= gsx_icp_normal_eq_scratch_bytes(ns), "gsx_icp_normal_eq_fwd: bad sizes");
-  const int nblk = (ns + kIcpBlock - 1) / kIcpBlock;
-  cudaStream_t s = (cudaStream_t)stream;
-  k_icp_linearize_idx<<<nblk, kIcpBlock, 0, s>>>(src_points, ns, nullptr, tgt_points, tgt_normals, 0, nn_idx,
-                                                 (float *)scratch);
-  k_icp_reduce_partials<<<1, 32, 0, s>>>((const float *)scratch, nblk, sums_out);
-  GSX_CHECK_LAUNCH("gsx_icp_normal_eq_fwd");
-  return 0;
-}
-
-extern "C" int gsx_icp_normal_eq_bwd(const float *src_points, int ns, const float *tgt_points,
-                                     const float *tgt_normals, const int64_t *nn_idx, const float *g_sums,
-                                     float *g_src, float *g_tgt_points_rows, float *g_tgt_normals_rows,
-                                     void *stream) {
-  GSX_CHECK_ARG(src_points && tgt_points && tgt_normals && nn_idx && g_sums && g_src && g_tgt_points_rows &&
-                    g_tgt_normals_rows,
-                "gsx_icp_normal_eq_bwd: null pointer");
-  GSX_CHECK_ARG(ns >= 1, "gsx_icp_normal_eq_bwd: bad sizes");
-  const int nblk = (ns + kIcpBlock - 1) / kIcpBlock;
-  k_icp_linearize_bwd<<<nblk, kIcpBlock, 0, (cudaStream_t)stream>>>(src_points, ns, nullptr, tgt_points, tgt_normals, 0,
-                                                                    nn_idx, g_sums, g_src, g_tgt_points_rows,
-                                                                    g_tgt_normals_rows);
-  GSX_CHECK_LAUNCH("gsx_icp_normal_eq_bwd");
-  return 0;
-}

@@ -244,15 +244,6 @@ extern "C" int gsx_icp_update_bwd(const float *xi, const float *err, const float
   return 0;
 }
 
-extern "C" int gsx_rigid_transform_fwd(const float *points, int64_t n, const float *T, float *out, void *stream) {
-  GSX_CHECK_ARG(n >= 0, "gsx_rigid_transform_fwd: negative count");
-  if (n == 0) return 0;
-  GSX_CHECK_ARG(points && T && out, "gsx_rigid_transform_fwd: null pointer");
-  k_rigid_fwd<<<(unsigned)((n + kRtBlock - 1) / kRtBlock), kRtBlock, 0, (cudaStream_t)stream>>>(points, n, nullptr, T, out);
-  GSX_CHECK_LAUNCH("gsx_rigid_transform_fwd");
-  return 0;
-}
-
 extern "C" int gsx_rigid_transform_batched_fwd(const float *points, const int32_t *counts, int64_t stride, int B,
                                                const float *T, float *out, void *stream) {
   GSX_CHECK_ARG(B >= 1 && stride >= 1, "gsx_rigid_transform_batched_fwd: bad sizes");
@@ -282,21 +273,4 @@ extern "C" int gsx_rigid_transform_batched_bwd(const float *points, const int32_
 extern "C" int64_t gsx_rigid_transform_bwd_scratch_bytes(int64_t n) {
   if (n < 0) return -1;
   return ((n + kRtBlock - 1) / kRtBlock) * 12 * 4 + 256;
-}
-
-extern "C" int gsx_rigid_transform_bwd(const float *points, int64_t n, const float *T, const float *g_out,
-                                       float *g_points, float *g_T, void *scratch, int64_t scratch_bytes,
-                                       void *stream) {
-  GSX_CHECK_ARG(n >= 0, "gsx_rigid_transform_bwd: negative count");
-  GSX_CHECK_ARG(T && g_T, "gsx_rigid_transform_bwd: null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int nblk = (int)((n + kRtBlock - 1) / kRtBlock);
-  if (n > 0) {
-    GSX_CHECK_ARG(points && g_out && g_points && scratch, "gsx_rigid_transform_bwd: null pointer");
-    GSX_CHECK_ARG(scratch_bytes >= gsx_rigid_transform_bwd_scratch_bytes(n), "gsx_rigid_transform_bwd: scratch too small");
-    k_rigid_bwd<<<nblk, kRtBlock, 0, st>>>(points, n, nullptr, T, g_out, g_points, (float *)scratch);
-  }
-  k_rigid_bwd_reduce<<<1, 32, 0, st>>>((const float *)scratch, nblk, g_T);
-  GSX_CHECK_LAUNCH("gsx_rigid_transform_bwd");
-  return 0;
 }

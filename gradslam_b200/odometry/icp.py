@@ -6,7 +6,7 @@ import torch
 
 from ..structures.pointclouds import Pointclouds
 from .base import OdometryProvider
-from .icputils import _taped_icp_batched, _wants_grad, icp_align
+from .icputils import _taped_icp, _wants_grad, icp_align
 
 __all__ = ["ICPOdometryProvider"]
 
@@ -31,18 +31,16 @@ def _provide(prov, maps_pc, frames_pc, mode):
     if _wants_grad(*frames_pc._grad_tensors(), *maps_pc._grad_tensors()):
         # differentiable mode: ONE chain of batched autograd ops for all elements (the reference's providers loop over
         # the batch in Python, odometry/icp.py:84-97)
-        T, _ = _taped_icp_batched(frames_pc.points_padded, frames_pc._counts_dev[frames_pc._cur], maps_pc.points_padded,
-                                  maps_pc.normals_padded, maps_pc._counts_dev[maps_pc._cur], None, mode, prov.numiters,
-                                  prov.damp, prov.dist_thresh, **kw)
+        T, _ = _taped_icp(frames_pc.points_padded, frames_pc._counts_dev[frames_pc._cur], maps_pc.points_padded,
+                          maps_pc.normals_padded, maps_pc._counts_dev[maps_pc._cur], None, mode, prov.numiters,
+                          prov.damp, prov.dist_thresh, **kw)
         return T.unsqueeze(1)
     # (the padded views are strided slices of the packed rows; the ICP kernels take dense (B,N,3) clouds)
     src = frames_pc.points_padded.contiguous()
     tgt, tgt_n = maps_pc.points_padded.contiguous(), maps_pc.normals_padded.contiguous()
     src_c = frames_pc._counts_dev[frames_pc._cur]
     tgt_c = maps_pc._counts_dev[maps_pc._cur]
-    T, _ = icp_align(src, src_c, tgt, tgt_n, tgt_c, None, mode, prov.numiters, prov.damp, prov.dist_thresh,
-                     lambda_max=getattr(prov, "lambda_max", 2.0), B=getattr(prov, "B", 1.0),
-                     B2=getattr(prov, "B2", 1.0), nu=getattr(prov, "nu", 200.0))
+    T, _ = icp_align(src, src_c, tgt, tgt_n, tgt_c, None, mode, prov.numiters, prov.damp, prov.dist_thresh, **kw)
     return T.unsqueeze(1)
 
 

@@ -164,149 +164,15 @@ def _wants_grad(*tensors):
     return torch.is_grad_enabled() and any(torch.is_tensor(t) and t.requires_grad for t in tensors)
 
 
+# The differentiable ICP loop is a chain of the autograd ops below on padded clouds (B, N, 3) with int32 sizes (B,):
+# one chain records all batch elements (the reference's providers run one chain per element, odometry/icp.py:84-97), and
+# a single cloud pair is a batch of one.  Padding rows contribute exact zeros to the fixed-order sums, so an element's
+# values do not depend on the padding or on the other elements.
 class _NormalEqFn(torch.autograd.Function):
-    """(src (Ns,3), tgt (Nt,3), tgt_normals (Nt,3), nn_idx (Ns,) int64) -> the 28 sums of the point-to-plane normal
-    equations.  forward = gsx_icp_normal_eq_fwd, backward = gsx_icp_normal_eq_bwd (hand-written kernels)."""
+    """(src (B,Ns,3), tgt (B,Nt,3), tgt_normals (B,Nt,3), nn_idx (B,Ns) int64, -1 = row unused, src sizes (B,) int32)
+    -> the 28 sums (B,28) of the point-to-plane normal equations.  forward = gsx_icp_normal_eq_batched_fwd,
+    backward = gsx_icp_normal_eq_batched_bwd (hand-written kernels; gradients w.r.t. src, tgt and tgt_normals)."""
 
-    @staticmethod
-    def forward(ctx, src, tgt, tgt_n, idx):
-        src_c, tgt_c, tn_c, idx_c = src.detach().contiguous(), tgt.detach().contiguous(), tgt_n.detach().contiguous(), \
-            idx.contiguous()
-        for name, t in (("src", src_c), ("tgt", tgt_c), ("tgt_normals", tn_c)):
-            _C.require_cuda(t, name)
-        ns, dev = src_c.shape[0], src_c.device
-        sums = torch.empty(28, dtype=torch.float32, device=dev)
-        lib = _C.lib()
-        nbytes = lib.gsx_icp_normal_eq_scratch_bytes(ns)
-        scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            rc = lib.gsx_icp_normal_eq_fwd(_C.ptr(src_c), ns, _C.ptr(tgt_c), _C.ptr(tn_c), _C.ptr(idx_c), _C.ptr(sums),
-                                           _C.ptr(scratch), nbytes, _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_normal_eq_fwd")
-        ctx.saved = (src_c, tgt_c, tn_c, idx_c)
-        return sums
-
-    @staticmethod
-    def backward(ctx, g):
-        src_c, tgt_c, tn_c, idx_c = ctx.saved
-        ns, dev = src_c.shape[0], src_c.device
-        g = g.contiguous().float()
-        g_src = torch.empty_like(src_c)
-        rows_p, rows_n = torch.empty_like(src_c), torch.empty_like(src_c)
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_icp_normal_eq_bwd(_C.ptr(src_c), ns, _C.ptr(tgt_c), _C.ptr(tn_c), _C.ptr(idx_c), _C.ptr(g),
-                                                _C.ptr(g_src), _C.ptr(rows_p), _C.ptr(rows_n), _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_normal_eq_bwd")
-        safe = idx_c.clamp(min=0)  # rows with idx < 0 carry zero gradients
-        g_tgt = torch.zeros_like(tgt_c).index_add_(0, safe, rows_p)
-        g_tn = torch.zeros_like(tn_c).index_add_(0, safe, rows_n)
-        return g_src, g_tgt, g_tn, None
-
-
-class _SolveFn(torch.autograd.Function):
-    """(28 sums, damp) -> (xi (6,), dT (4,4)): damped 6x6 solve + se3_exp in one kernel (K7a).
-    forward = gsx_icp_solve_fwd, backward = gsx_icp_solve_bwd (dual numbers, one lane per input)."""
-
-    @staticmethod
-    def forward(ctx, sums, damp):
-        s, d = sums.detach().contiguous().float(), damp.detach().reshape(1).contiguous().float()
-        _C.require_cuda(s, "sums")
-        dev = s.device
-        xi = torch.empty(6, dtype=torch.float32, device=dev)
-        dT = torch.empty((4, 4), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_icp_solve_fwd(_C.ptr(s), _C.ptr(d), 1, _C.ptr(xi), _C.ptr(dT), _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_solve_fwd")
-        ctx.saved = (s, d, damp.shape)
-        return xi, dT
-
-    @staticmethod
-    def backward(ctx, g_xi, g_dT):
-        s, d, damp_shape = ctx.saved
-        dev = s.device
-        g_xi = None if g_xi is None else g_xi.contiguous().float()
-        g_dT = None if g_dT is None else g_dT.contiguous().float()
-        g_s, g_d = torch.empty_like(s), torch.empty_like(d)
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_icp_solve_bwd(_C.ptr(s), _C.ptr(d), 1, _C.ptr(g_xi), _C.ptr(g_dT), _C.ptr(g_s),
-                                            _C.ptr(g_d), _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_solve_bwd")
-        return g_s, g_d.view(damp_shape)
-
-
-class _UpdateFn(torch.autograd.Function):
-    """(xi, err, new_err, damp, T) -> (new damp, applied step (4,4), step @ T): LM accept / reject (mode 0) or the
-    gradLM gates (mode 1), the applied se3_exp and the pose accumulation in one kernel (K7b).
-    forward = gsx_icp_update_fwd, backward = gsx_icp_update_bwd."""
-
-    @staticmethod
-    def forward(ctx, xi, err, new_err, damp, T, mode, lambda_max, B, B2, nu):
-        dev = xi.device
-        ins = [t.detach().reshape(n).contiguous().float() for t, n in ((xi, 6), (err, 1), (new_err, 1), (damp, 1),
-                                                                       (T, 16))]
-        _C.require_cuda(ins[0], "xi")
-        damp_out = torch.empty(1, dtype=torch.float32, device=dev)
-        dT = torch.empty((4, 4), dtype=torch.float32, device=dev)
-        Tn = torch.empty((4, 4), dtype=torch.float32, device=dev)
-        par = (int(mode), float(lambda_max), float(B), float(B2), float(nu))
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_icp_update_fwd(*[_C.ptr(t) for t in ins], 1, *par, _C.ptr(damp_out), _C.ptr(dT),
-                                             _C.ptr(Tn), _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_update_fwd")
-        ctx.saved = (ins, par, (xi.shape, err.shape, new_err.shape, damp.shape, T.shape))
-        return damp_out.view(damp.shape), dT, Tn
-
-    @staticmethod
-    def backward(ctx, g_damp, g_dT, g_T):
-        ins, par, shapes = ctx.saved
-        dev = ins[0].device
-        gs = [None if g is None else g.contiguous().float() for g in (g_damp, g_dT, g_T)]
-        outs = [torch.empty_like(t) for t in ins]
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_icp_update_bwd(*[_C.ptr(t) for t in ins], 1, *par, *[_C.ptr(g) for g in gs],
-                                             *[_C.ptr(o) for o in outs], _C.stream_ptr(dev))
-        _C.check(rc, "gsx_icp_update_bwd")
-        return tuple(o.view(sh) for o, sh in zip(outs, shapes)) + (None,) * 5
-
-
-class _RigidTransformFn(torch.autograd.Function):
-    """(points (N,3), T (4,4)) -> R p + t (transform_pointcloud, geometryutils.py:737-794).
-    forward = gsx_rigid_transform_fwd, backward = gsx_rigid_transform_bwd (deterministic reduction for d/dT)."""
-
-    @staticmethod
-    def forward(ctx, points, T):
-        p, Tc = points.detach().contiguous().float(), T.detach().contiguous().float()
-        _C.require_cuda(p, "points")
-        dev = p.device
-        out = torch.empty_like(p)
-        with torch.cuda.device(dev):
-            rc = _C.lib().gsx_rigid_transform_fwd(_C.ptr(p), p.shape[0], _C.ptr(Tc), _C.ptr(out), _C.stream_ptr(dev))
-        _C.check(rc, "gsx_rigid_transform_fwd")
-        ctx.saved = (p, Tc)
-        return out
-
-    @staticmethod
-    def backward(ctx, g):
-        p, Tc = ctx.saved
-        dev, n = p.device, p.shape[0]
-        g = g.contiguous().float()
-        g_p, g_T = torch.empty_like(p), torch.empty_like(Tc)
-        lib = _C.lib()
-        nbytes = lib.gsx_rigid_transform_bwd_scratch_bytes(n)
-        scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            rc = lib.gsx_rigid_transform_bwd(_C.ptr(p), n, _C.ptr(Tc), _C.ptr(g), _C.ptr(g_p), _C.ptr(g_T),
-                                             _C.ptr(scratch), nbytes, _C.stream_ptr(dev))
-        _C.check(rc, "gsx_rigid_transform_bwd")
-        return g_p, g_T
-
-
-# ------------------------------------------------------------------------------------------------ batched variants
-# The same four ops for a padded batch (B, N, 3) with int32 sizes: ONE op chain records the differentiable ICP of all
-# batch elements (the reference's providers, and round 1 here, ran one chain per element: odometry/icp.py:84-97).  Every
-# kernel takes the batch index from blockIdx.y; values per element are bit-identical to the per-element ops (padding rows
-# contribute exact zeros to the fixed-order sums).
-class _NormalEqBatchedFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, src, tgt, tgt_n, idx, src_counts):
         src_c, tgt_c, tn_c = (t.detach().contiguous().float() for t in (src, tgt, tgt_n))
@@ -346,7 +212,10 @@ class _NormalEqBatchedFn(torch.autograd.Function):
         return g_src, g_tgt.view(Bn, Nt, 3), g_tn.view(Bn, Nt, 3), None, None
 
 
-class _SolveBatchedFn(torch.autograd.Function):
+class _SolveFn(torch.autograd.Function):
+    """(sums (B,28), damp (B,)) -> (xi (B,6), dT (B,4,4)): damped 6x6 solve + se3_exp in one kernel (K7a).
+    forward = gsx_icp_solve_fwd, backward = gsx_icp_solve_bwd (dual numbers, one lane per input)."""
+
     @staticmethod
     def forward(ctx, sums, damp):
         s, d = sums.detach().contiguous().float(), damp.detach().contiguous().float()
@@ -374,7 +243,11 @@ class _SolveBatchedFn(torch.autograd.Function):
         return g_s, g_d
 
 
-class _UpdateBatchedFn(torch.autograd.Function):
+class _UpdateFn(torch.autograd.Function):
+    """(xi (B,6), err (B,), new_err (B,), damp (B,), T (B,4,4)) -> (new damp, applied step (B,4,4), step @ T): LM
+    accept / reject (mode 0) or the gradLM gates (mode 1), the applied se3_exp and the pose accumulation in one kernel
+    (K7b).  forward = gsx_icp_update_fwd, backward = gsx_icp_update_bwd."""
+
     @staticmethod
     def forward(ctx, xi, err, new_err, damp, T, mode, lambda_max, B, B2, nu):
         dev = xi.device
@@ -405,7 +278,11 @@ class _UpdateBatchedFn(torch.autograd.Function):
         return tuple(outs) + (None,) * 5
 
 
-class _RigidTransformBatchedFn(torch.autograd.Function):
+class _RigidTransformFn(torch.autograd.Function):
+    """(points (B,N,3), T (B,4,4), sizes (B,) int32) -> R p + t (transform_pointcloud, geometryutils.py:737-794), zero
+    on padding rows.  forward = gsx_rigid_transform_batched_fwd, backward = gsx_rigid_transform_batched_bwd
+    (deterministic reduction for d/dT)."""
+
     @staticmethod
     def forward(ctx, points, T, counts):
         p, Tc = points.detach().contiguous().float(), T.detach().contiguous().float()
@@ -436,79 +313,52 @@ class _RigidTransformBatchedFn(torch.autograd.Function):
         return g_p, g_T, None
 
 
-def _normal_equations_batched(src, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, target_cache=None):
+def _normal_equations(src, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, target_cache=None):
+    """Association (CUDA exact 1-NN, index-only) + the differentiable normal-equation op -> ((B,28) sums, idx)."""
     d2, idx = knn1(src.detach(), tgt.detach(), src_counts, tgt_counts, target_cache)
     if dist_thresh is not None:
         idx = torch.where(d2 < dist_thresh, idx, torch.full_like(idx, -1))
-    return _NormalEqBatchedFn.apply(src, tgt, tgt_n, idx, src_counts), idx
+    return _NormalEqFn.apply(src, tgt, tgt_n, idx, src_counts), idx
 
 
-def _taped_icp_batched(src, src_counts, tgt, tgt_n, tgt_counts, T0, mode, numiters, damp, dist_thresh, lambda_max=2.0,
-                       B=1.0, B2=1.0, nu=200.0):
-    """The differentiable ICP / gradICP loop of `_taped_icp` for a padded batch: src (Bn,Ns,3), tgt / tgt_n (Bn,Nt,3),
-    int32 sizes (Bn,).  One chain of batched ops for all elements; returns (T (Bn,4,4), last nn idx (Bn,Ns), -1 = none).
-    Per element the values are bit-identical to the per-element chain and to the fused no-grad loop."""
+def _taped_icp(src, src_counts, tgt, tgt_n, tgt_counts, T0, mode, numiters, damp, dist_thresh, lambda_max=2.0, B=1.0,
+               B2=1.0, nu=200.0):
+    """Differentiable ICP / gradICP, used when an input requires grad: the same loop as the fused kernel sequence, as a
+    chain of autograd ops that each have a hand-written forward AND backward kernel - rigid transform
+    (`_RigidTransformFn`), 1-NN association (index-only, no gradient, as in the reference), normal equations
+    (`_NormalEqFn`), damped solve + se3_exp (`_SolveFn`), LM / gradLM update (`_UpdateFn`).  PyTorch only records the
+    tape; no ATen arithmetic runs between the ops and there is no host synchronisation (icputils.py:235-545).
+    src (Bn,Ns,3), tgt / tgt_n (Bn,Nt,3), int32 sizes (Bn,), T0 (1,4,4), (Bn,4,4) or None.  Returns (T (Bn,4,4), last nn
+    idx (Bn,Ns), -1 = none); per element the poses are bit-identical to the fused no-grad loop."""
     dev = src.device
     Bn = src.shape[0]
     dampt = torch.full((Bn,), float(damp), dtype=torch.float32, device=dev)
     T = (torch.eye(4, dtype=torch.float32, device=dev).repeat(Bn, 1, 1) if T0 is None
          else T0.to(torch.float32).expand(Bn, 4, 4).contiguous())
     tgt, tgt_n = tgt.contiguous(), tgt_n.contiguous()  # once (strided views of packed map rows), not per iteration
-    cur = _RigidTransformBatchedFn.apply(src, T, src_counts)
+    cur = _RigidTransformFn.apply(src, T, src_counts)
     idx = None
     grid = {}  # the target's search grid: built by the first of the 2 * numiters associations
     for _ in range(numiters):
-        sums, idx = _normal_equations_batched(cur, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, grid)
-        xi, dT = _SolveBatchedFn.apply(sums, dampt)
-        one_step = _RigidTransformBatchedFn.apply(cur, dT, src_counts)
-        sums_next, _ = _normal_equations_batched(one_step, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, grid)
-        dampt, dT_applied, T = _UpdateBatchedFn.apply(xi, sums[:, 27], sums_next[:, 27], dampt, T, mode, lambda_max, B,
-                                                      B2, nu)
-        cur = _RigidTransformBatchedFn.apply(cur, dT_applied, src_counts)
+        sums, idx = _normal_equations(cur, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, grid)
+        xi, dT = _SolveFn.apply(sums, dampt)
+        one_step = _RigidTransformFn.apply(cur, dT, src_counts)
+        sums_next, _ = _normal_equations(one_step, src_counts, tgt, tgt_n, tgt_counts, dist_thresh, grid)
+        dampt, dT_applied, T = _UpdateFn.apply(xi, sums[:, 27], sums_next[:, 27], dampt, T, mode, lambda_max, B, B2, nu)
+        cur = _RigidTransformFn.apply(cur, dT_applied, src_counts)
     return T, idx
 
 
-def _normal_equations(src, tgt, tgt_n, dist_thresh):
-    """Association (CUDA exact 1-NN, index-only) + the differentiable normal-equation op.  src (Ns,3) -> 28 sums."""
-    d2, idx = knn1(src.detach().unsqueeze(0), tgt.detach().unsqueeze(0))
-    idx = idx[0]
-    if dist_thresh is not None:
-        idx = torch.where(d2[0] < dist_thresh, idx, torch.full_like(idx, -1))
-    return _NormalEqFn.apply(src, tgt, tgt_n, idx), idx
-
-
-def _taped_icp(src_pc, tgt_pc, tgt_normals, initial_transform, mode, numiters, damp, dist_thresh, lambda_max=2.0,
-               B=1.0, B2=1.0, nu=200.0):
-    """Differentiable variant used when an input requires grad: the same loop as the fused kernel sequence, as a chain
-    of autograd ops that each have a hand-written forward AND backward kernel -
-    rigid transform (`_RigidTransformFn`), 1-NN association (index-only, no gradient, as in the reference), normal
-    equations (`_NormalEqFn`), damped solve + se3_exp (`_SolveFn`), LM / gradLM update (`_UpdateFn`).  PyTorch only
-    records the tape; no ATen arithmetic runs between the ops and there is no host synchronisation
-    (icputils.py:235-545)."""
-    dtype, device = torch.float32, src_pc.device
-    damp = torch.tensor([float(damp)], dtype=dtype, device=device)
-    T = torch.eye(4, dtype=dtype, device=device) if initial_transform is None else initial_transform.to(dtype)
-    src = _RigidTransformFn.apply(src_pc[0], T)
-    tgt, tgt_n = tgt_pc[0], tgt_normals[0]
-    idx = None
-    for _ in range(numiters):
-        sums, idx = _normal_equations(src, tgt, tgt_n, dist_thresh)
-        xi, dT = _SolveFn.apply(sums, damp)
-        one_step = _RigidTransformFn.apply(src, dT)
-        sums_next, _ = _normal_equations(one_step, tgt, tgt_n, dist_thresh)
-        damp, dT_applied, T = _UpdateFn.apply(xi, sums[27], sums_next[27], damp, T, mode, lambda_max, B, B2, nu)
-        src = _RigidTransformFn.apply(src, dT_applied)
-    return T, idx[idx >= 0]
-
-
 def _single(src_pc, tgt_pc, tgt_normals, initial_transform, mode, numiters, damp, dist_thresh, **kw):
-    if _wants_grad(src_pc, tgt_pc, tgt_normals, initial_transform):
-        return _taped_icp(src_pc, tgt_pc, tgt_normals, initial_transform, mode, numiters, damp, dist_thresh, **kw)
+    """One cloud pair as a batch of one: the taped op chain when an input requires grad, else the fused loop."""
     dev = src_pc.device
     T0 = None if initial_transform is None else initial_transform.view(1, 4, 4)
-    T, idx = icp_align(src_pc.contiguous(), _counts(src_pc.shape[1], 1, dev), tgt_pc.contiguous(),
-                       tgt_normals.contiguous(), _counts(tgt_pc.shape[1], 1, dev), T0, mode, numiters, damp,
-                       dist_thresh, want_idx=True, **kw)
+    args = (src_pc.contiguous(), _counts(src_pc.shape[1], 1, dev), tgt_pc.contiguous(), tgt_normals.contiguous(),
+            _counts(tgt_pc.shape[1], 1, dev), T0, mode, numiters, damp, dist_thresh)
+    if _wants_grad(src_pc, tgt_pc, tgt_normals, initial_transform):
+        T, idx = _taped_icp(*args, **kw)
+    else:
+        T, idx = icp_align(*args, want_idx=True, **kw)
     idx = idx[0]
     return T[0], idx[idx >= 0]
 

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define GSX_VERSION 200 /* 0.2.0: sector-packed map rows, per-frame records */
+#define GSX_VERSION 201 /* 0.2.1: single-cloud gsx_icp_normal_eq_fwd/bwd, gsx_rigid_transform_fwd/bwd removed */
 
 int gsx_version(void);
 const char *gsx_last_error(void);
@@ -258,32 +258,17 @@ int gsx_knn1(const float *src_points, const int32_t *src_count, int ns_stride, c
              const int32_t *tgt_count, int nt_stride, int B, int64_t *idx_out, float *d2_out, void *scratch,
              int64_t scratch_bytes, int build_grid, void *stream);
 
-/* K6 as a differentiable op: for a GIVEN association nn_idx (int64 (ns), -1 = row unused) reduce the point-to-plane
- * rows A_i = [n, s x n], r_i = n.(p - s) (gauss_newton_solve, icputils.py:210-230) to the 28 sums
+/* K6 as a differentiable op on padded clouds (B, stride, 3) with int32 sizes (NULL = all rows): for a GIVEN
+ * association nn_idx (int64 (B, ns_stride), -1 = row unused) reduce the point-to-plane rows A_i = [n, s x n],
+ * r_i = n.(p - s) (gauss_newton_solve, icputils.py:210-230) to the 28 sums (B,28)
  * [upper triangle of A^T A (21, row-major), A^T r (6), r^T r] (the matmuls of solve_linear_system, icputils.py:85-90).
- * Backward: from d(loss)/d(sums) the gradient w.r.t. every source point (ns,3) and, per SOURCE row, w.r.t. its
- * associated target point and normal (ns,3 each; the caller scatter-adds them through nn_idx).  Single clouds
- * (B = 1), deterministic, no atomics.  scratch: gsx_icp_normal_eq_scratch_bytes(ns) bytes. */
+ * Backward: from d(loss)/d(sums) the gradient w.r.t. every source point (B, ns_stride, 3) and, per SOURCE row,
+ * w.r.t. its associated target point and normal (B, ns_stride, 3 each; the caller scatter-adds them through nn_idx).
+ * One launch for all elements (the differentiable mode's op chain is recorded ONCE for the batch instead of once per
+ * element, which is what the reference's providers do, odometry/icp.py:84-97); a single cloud is B = 1.  Padding rows
+ * get zero outputs / zero gradients.  Deterministic, no atomics.
+ * scratch: B * gsx_icp_normal_eq_scratch_bytes(ns_stride) bytes. */
 int64_t gsx_icp_normal_eq_scratch_bytes(int ns);
-int gsx_icp_normal_eq_fwd(const float *src_points, int ns, const float *tgt_points, const float *tgt_normals,
-                          const int64_t *nn_idx, float *sums_out, void *scratch, int64_t scratch_bytes, void *stream);
-int gsx_icp_normal_eq_bwd(const float *src_points, int ns, const float *tgt_points, const float *tgt_normals,
-                          const int64_t *nn_idx, const float *g_sums, float *g_src, float *g_tgt_points_rows,
-                          float *g_tgt_normals_rows, void *stream);
-
-/* K7 as differentiable ops (n independent problems; every array is dense float32, device):
- * _solve_: xi = (A^T A + damp I)^-1 A^T b from the 28 sums of gsx_icp_normal_eq_fwd and damp (n), then dT = se3_exp(xi).
- *          replaces solve_linear_system   gradslam/odometry/icputils.py:22-90  and  se3_exp  geometry/se3utils.py:77-115
- * _update_: mode 0 = LM accept / reject (icputils.py:356-365): new_err < err -> applied step se3_exp(xi), damp / 2,
- *          else identity, damp * 2;  mode 1 = gradLM gates (icputils.py:519-543): diff = clamp(new_err - err, +-70),
- *          damp * (1/lambda_max + (lambda_max - 1/lambda_max) / (1 + exp(-B diff))), applied step
- *          se3_exp(xi / (1 + exp(-B2 diff))^(1/nu)).  Outputs: new damp (n), applied step (n,16), T_out = step * T (n,16).
- * The backward entries take the forward inputs again plus the upstream gradients (any may be NULL = zero) and write
- * the gradient of every forward input (same arithmetic evaluated on dual numbers, one lane per input). */
-/* the same two ops for a padded batch (B, stride, 3) with int32 sizes (NULL = all rows): one launch for all elements
- * (the differentiable mode's op chain is recorded ONCE for the batch instead of once per element, which is what the
- * reference's providers do, odometry/icp.py:84-97).  sums (B,28); nn_idx (B, ns_stride), -1 = no neighbour; the target
- * gradients come back per SOURCE row (B, ns_stride, 3).  Padding rows get zero outputs / zero gradients. */
 int gsx_icp_normal_eq_batched_fwd(const float *src_points, const int32_t *src_count, int ns_stride,
                                   const float *tgt_points, const float *tgt_normals, int nt_stride, int B,
                                   const int64_t *nn_idx, float *sums_out, void *scratch, int64_t scratch_bytes,
@@ -292,6 +277,17 @@ int gsx_icp_normal_eq_batched_bwd(const float *src_points, const int32_t *src_co
                                   const float *tgt_points, const float *tgt_normals, int nt_stride, int B,
                                   const int64_t *nn_idx, const float *g_sums, float *g_src, float *g_tgt_points_rows,
                                   float *g_tgt_normals_rows, void *stream);
+
+/* K7 as differentiable ops (n independent problems; every array is dense float32, device):
+ * _solve_: xi = (A^T A + damp I)^-1 A^T b from the 28 sums of gsx_icp_normal_eq_batched_fwd and damp (n), then
+ *          dT = se3_exp(xi).
+ *          replaces solve_linear_system   gradslam/odometry/icputils.py:22-90  and  se3_exp  geometry/se3utils.py:77-115
+ * _update_: mode 0 = LM accept / reject (icputils.py:356-365): new_err < err -> applied step se3_exp(xi), damp / 2,
+ *          else identity, damp * 2;  mode 1 = gradLM gates (icputils.py:519-543): diff = clamp(new_err - err, +-70),
+ *          damp * (1/lambda_max + (lambda_max - 1/lambda_max) / (1 + exp(-B diff))), applied step
+ *          se3_exp(xi / (1 + exp(-B2 diff))^(1/nu)).  Outputs: new damp (n), applied step (n,16), T_out = step * T (n,16).
+ * The backward entries take the forward inputs again plus the upstream gradients (any may be NULL = zero) and write
+ * the gradient of every forward input (same arithmetic evaluated on dual numbers, one lane per input). */
 int gsx_icp_solve_fwd(const float *sums, const float *damp, int n, float *xi_out, float *dT_out, void *stream);
 int gsx_icp_solve_bwd(const float *sums, const float *damp, int n, const float *g_xi, const float *g_dT,
                       float *g_sums, float *g_damp, void *stream);
@@ -303,18 +299,16 @@ int gsx_icp_update_bwd(const float *xi, const float *err, const float *new_err, 
                        const float *g_dT_out, const float *g_T_out, float *g_xi, float *g_err, float *g_new_err,
                        float *g_damp, float *g_T, void *stream);
 
-/* out = R p + t for a cloud (n,3) and one 4x4 T; backward: g_points = R^T g, g_T = sum_i g_i (x) [p_i; 1] (fixed-order
- * reduction; bottom row zero).     replaces transform_pointcloud   gradslam/geometry/geometryutils.py:737-794 */
-int gsx_rigid_transform_fwd(const float *points, int64_t n, const float *T, float *out, void *stream);
+/* out = R p + t for padded clouds points (B, stride, 3) with int32 sizes counts (B) (NULL = all rows) and T (B,4,4);
+ * padding rows are written as zeros.  backward: g_points = R^T g (zero on padding rows), g_T = sum_i g_i (x) [p_i; 1]
+ * (fixed-order reduction; bottom row zero).  scratch: B * gsx_rigid_transform_bwd_scratch_bytes(stride) bytes.
+ *          replaces transform_pointcloud   gradslam/geometry/geometryutils.py:737-794 */
 int64_t gsx_rigid_transform_bwd_scratch_bytes(int64_t n);
-/* batched: points (B, stride, 3), T (B,4,4); scratch B * gsx_rigid_transform_bwd_scratch_bytes(stride) bytes */
 int gsx_rigid_transform_batched_fwd(const float *points, const int32_t *counts, int64_t stride, int B, const float *T,
                                     float *out, void *stream);
 int gsx_rigid_transform_batched_bwd(const float *points, const int32_t *counts, int64_t stride, int B, const float *T,
                                     const float *g_out, float *g_points, float *g_T, void *scratch,
                                     int64_t scratch_bytes, void *stream);
-int gsx_rigid_transform_bwd(const float *points, int64_t n, const float *T, const float *g_out, float *g_points,
-                            float *g_T, void *scratch, int64_t scratch_bytes, void *stream);
 
 /* full ICP / gradICP on given clouds.  initial_transform (B,16) or NULL (identity).  transform_out (B,16).
  * nn_idx_out optional int64 (B, ns_stride): association of the last iteration (-1 = filtered out).

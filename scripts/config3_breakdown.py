@@ -73,7 +73,7 @@ print(prof.key_averages().table(sort_by="self_cuda_time_total", row_limit=20, ma
 wrap(icputils, "downsample_rgbdimages")
 wrap(icputils, "downsample_pointclouds")
 wrap(fusionutils, "find_active_map_points")
-wrap(icp_mod, "_taped_icp_batched")
+wrap(icp_mod, "_taped_icp")
 wrap(icputils, "knn1")
 wrap(fusionutils, "update_map_aggregate")
 wrap(icpslam, "update_map_aggregate", "update_map_aggregate(icpslam)")

@@ -27,7 +27,7 @@ def test_library_exports_every_declared_symbol():
 
 def test_host_only_entry_points():
     lib = _C.lib()
-    assert lib.gsx_version() == 200
+    assert lib.gsx_version() == 201
     n = lib.gsx_fusion_workspace_bytes(8, 480, 640)
     assert n >= 8 * 480 * 640 * 16
     assert 0 < lib.gsx_fusion_workspace_stats_offset(8, 480, 640) < n

@@ -89,8 +89,9 @@ def test_backward_only_global_maps_and_no_pose_grad():
 
 
 def test_gradicp_function_gradients_match_oracle_autograd():
-    """point_to_plane_gradICP in differentiable mode (CUDA 1-NN + taped algebra): d(T)/d(src) equals the gradient
-    PyTorch's tape gives for the oracle restatement of the reference (icputils.py:370-545)."""
+    """point_to_plane_gradICP in differentiable mode (CUDA 1-NN + taped algebra): d(T)/d(src) and
+    d(T)/d(initial_transform) equal the gradients PyTorch's tape gives for the oracle restatement of the reference
+    (icputils.py:370-545)."""
     import gsx_oracle as oracle
     from gradslam_b200.odometry import icputils
 
@@ -102,17 +103,17 @@ def test_gradicp_function_gradients_match_oracle_autograd():
     src0 = oracle.rigid_apply(T_true, tgt)
     w = torch.randn(4, 4, generator=torch.Generator().manual_seed(1))
     # oracle (CPU autograd)
-    s_ref = src0.clone().requires_grad_(True)
-    T_ref, _ = oracle.point_to_plane_gradicp(s_ref, tgt, tgt_n, torch.eye(4), numiters=4)
+    s_ref, t_ref = src0.clone().requires_grad_(True), torch.eye(4).requires_grad_(True)
+    T_ref, _ = oracle.point_to_plane_gradicp(s_ref, tgt, tgt_n, t_ref, numiters=4)
     (T_ref * w).sum().backward()
     # engine, differentiable mode
-    s_gpu = src0.clone().to(DEV).requires_grad_(True)
-    T_gpu, _ = icputils.point_to_plane_gradICP(s_gpu[None], tgt[None].to(DEV), tgt_n[None].to(DEV),
-                                               torch.eye(4, device=DEV), numiters=4)
+    s_gpu, t_gpu = src0.clone().to(DEV).requires_grad_(True), torch.eye(4, device=DEV).requires_grad_(True)
+    T_gpu, _ = icputils.point_to_plane_gradICP(s_gpu[None], tgt[None].to(DEV), tgt_n[None].to(DEV), t_gpu, numiters=4)
     (T_gpu * w.to(DEV)).sum().backward()
     torch.testing.assert_close(T_gpu.detach().cpu(), T_ref.detach(), rtol=0, atol=1e-4)
-    scale = s_ref.grad.abs().max().item()
-    torch.testing.assert_close(s_gpu.grad.cpu(), s_ref.grad, rtol=2e-2, atol=2e-3 * scale)
+    for got, want in ((s_gpu.grad, s_ref.grad), (t_gpu.grad, t_ref.grad)):
+        scale = want.abs().max().item()
+        torch.testing.assert_close(got.cpu(), want, rtol=2e-2, atol=2e-3 * scale)
     # the fused (non-differentiable) loop gives the same forward value
     T_fused, _ = icputils.point_to_plane_gradICP(src0[None].to(DEV), tgt[None].to(DEV), tgt_n[None].to(DEV),
                                                  torch.eye(4, device=DEV), numiters=4)
@@ -266,8 +267,8 @@ def test_solve_update_transform_ops_forward_and_backward():
     o_ref = refm._solve(torch.cat([s_ref, d_ref]))
     (o_ref * wo).sum().backward()
     s_gpu, d_gpu = sums64.float().to(DEV).requires_grad_(True), damp64.float().to(DEV).requires_grad_(True)
-    xi, dT = iu._SolveFn.apply(s_gpu, d_gpu)
-    torch.testing.assert_close(torch.cat([xi, dT.reshape(-1)]).detach().cpu().double(), o_ref.detach(), rtol=0, atol=2e-6)
+    xi, dT = iu._SolveFn.apply(s_gpu[None], d_gpu)  # a batch of one problem
+    torch.testing.assert_close(torch.cat([xi[0], dT.reshape(-1)]).detach().cpu().double(), o_ref.detach(), rtol=0, atol=2e-6)
     ((xi * wo[:6].float().to(DEV)).sum() + (dT.reshape(-1) * wo[6:].float().to(DEV)).sum()).backward()
     for got, want in ((s_gpu.grad, s_ref.grad), (d_gpu.grad, d_ref.grad)):
         torch.testing.assert_close(got.cpu().double(), want, rtol=1e-3, atol=2e-4 * s_ref.grad.abs().max().item())
@@ -279,8 +280,8 @@ def test_solve_update_transform_ops_forward_and_backward():
         wu = torch.randn(33, dtype=torch.float64, generator=g)
         o_ref = refm._update(inp, mode, 2.0, 1.0, 1.0, 200.0)
         (o_ref * wu).sum().backward()
-        leaf = [t.float().to(DEV).requires_grad_(True) for t in (xi64, torch.tensor(err), torch.tensor(nerr),
-                                                                  torch.tensor([1e-3]), T64)]
+        leaf = [t.float().to(DEV).requires_grad_(True) for t in (xi64[None], torch.tensor([err]), torch.tensor([nerr]),
+                                                                  torch.tensor([1e-3]), T64[None])]
         dmp, dTa, Tn = iu._UpdateFn.apply(*leaf, mode, 2.0, 1.0, 1.0, 200.0)
         got = torch.cat([dmp.reshape(-1), dTa.reshape(-1), Tn.reshape(-1)])
         torch.testing.assert_close(got.detach().cpu().double(), o_ref.detach(), rtol=0, atol=2e-6)
@@ -293,12 +294,12 @@ def test_solve_update_transform_ops_forward_and_backward():
     wp = torch.randn(1000, 3, dtype=torch.float64, generator=g)
     p_ref, t_ref = P64.clone().requires_grad_(True), T64.clone().requires_grad_(True)
     ((p_ref @ t_ref[:3, :3].t() + t_ref[:3, 3]) * wp).sum().backward()
-    p_gpu, t_gpu = P64.float().to(DEV).requires_grad_(True), T64.float().to(DEV).requires_grad_(True)
-    out = iu._RigidTransformFn.apply(p_gpu, t_gpu)
-    torch.testing.assert_close(out.detach().cpu().double(), (P64 @ T64[:3, :3].t() + T64[:3, 3]), rtol=0, atol=1e-5)
-    (out * wp.float().to(DEV)).sum().backward()
-    torch.testing.assert_close(p_gpu.grad.cpu().double(), p_ref.grad, rtol=1e-4, atol=1e-5)
-    torch.testing.assert_close(t_gpu.grad.cpu().double(), t_ref.grad, rtol=1e-4, atol=1e-3)
+    p_gpu, t_gpu = P64[None].float().to(DEV).requires_grad_(True), T64[None].float().to(DEV).requires_grad_(True)
+    out = iu._RigidTransformFn.apply(p_gpu, t_gpu, torch.tensor([1000], dtype=torch.int32, device=DEV))
+    torch.testing.assert_close(out[0].detach().cpu().double(), (P64 @ T64[:3, :3].t() + T64[:3, 3]), rtol=0, atol=1e-5)
+    (out[0] * wp.float().to(DEV)).sum().backward()
+    torch.testing.assert_close(p_gpu.grad[0].cpu().double(), p_ref.grad, rtol=1e-4, atol=1e-5)
+    torch.testing.assert_close(t_gpu.grad[0].cpu().double(), t_ref.grad, rtol=1e-4, atol=1e-3)
 
 
 def test_icp_lm_function_gradients_match_oracle_autograd():
@@ -353,19 +354,21 @@ def test_normal_equation_op_forward_and_backward():
     a = [t.clone().double().requires_grad_(True) for t in (src, tgt, tn)]
     want = ref(*a)
     (want * w.double()).sum().backward()
-    b_ = [t.clone().to(DEV).requires_grad_(True) for t in (src, tgt, tn)]
-    got = _NormalEqFn.apply(b_[0], b_[1], b_[2], idx.to(DEV))
-    torch.testing.assert_close(got.cpu().double(), want.detach(), rtol=1e-4, atol=1e-3)
-    (got * w.to(DEV)).sum().backward()
+    b_ = [t[None].clone().to(DEV).requires_grad_(True) for t in (src, tgt, tn)]  # a batch of one cloud pair
+    got = _NormalEqFn.apply(b_[0], b_[1], b_[2], idx[None].to(DEV), torch.tensor([ns], dtype=torch.int32, device=DEV))
+    torch.testing.assert_close(got[0].cpu().double(), want.detach(), rtol=1e-4, atol=1e-3)
+    (got[0] * w.to(DEV)).sum().backward()
     for x, y in zip(b_, a):
         scale = y.grad.abs().max().item()
-        torch.testing.assert_close(x.grad.cpu().double(), y.grad, rtol=1e-3, atol=1e-4 * scale)
+        torch.testing.assert_close(x.grad[0].cpu().double(), y.grad, rtol=1e-3, atol=1e-4 * scale)
 
 
-def test_batched_differentiable_icp_equals_per_element_chain():
-    """The batched op chain (one set of autograd ops for all elements, ragged sizes) against the per-element chain of
-    round 1: transforms bit-identical, association identical, gradients w.r.t. the source clouds, the target clouds and
-    the target normals equal to float32 rounding; and the providers use it (ICPSLAM-style call with B=3)."""
+def test_batched_differentiable_icp_equals_single_element_runs():
+    """The differentiable op chain on a padded batch (one set of autograd ops for all elements, ragged sizes) against
+    each element alone through the public point_to_plane_gradICP: transforms bit-identical, association identical,
+    gradients w.r.t. the source clouds, the target clouds and the target normals equal to float32 rounding, so an
+    element's result depends neither on the padding nor on the other elements; and the providers use the chain
+    (ICPSLAM-style call with B=3)."""
     import gradslam_b200 as gs
     from gradslam_b200.odometry import icputils as iu
     from gradslam_b200.odometry.gradicp import GradICPOdometryProvider
@@ -392,12 +395,12 @@ def test_batched_differentiable_icp_equals_per_element_chain():
     ct = torch.tensor(sizes_t, dtype=torch.int32, device=DEV)
     w = torch.randn(Bn, 4, 4, generator=g).to(DEV)
     leaves = [t.clone().requires_grad_(True) for t in (src, tgt, tgt_n)]
-    T_b, idx_b = iu._taped_icp_batched(leaves[0], cs, leaves[1], leaves[2], ct, None, 1, 4, 1e-8, None)
+    T_b, idx_b = iu._taped_icp(leaves[0], cs, leaves[1], leaves[2], ct, None, 1, 4, 1e-8, None)
     (T_b * w).sum().backward()
     for b in range(Bn):
         l1 = [src[b:b + 1, : sizes_s[b]].clone().requires_grad_(True), tgt[b:b + 1, : sizes_t[b]].clone().requires_grad_(True),
               tgt_n[b:b + 1, : sizes_t[b]].clone().requires_grad_(True)]
-        T_1, idx_1 = iu._taped_icp(l1[0], l1[1], l1[2], None, 1, 4, 1e-8, None)
+        T_1, idx_1 = iu.point_to_plane_gradICP(l1[0], l1[1], l1[2], numiters=4, damp=1e-8)
         (T_1 * w[b]).sum().backward()
         assert torch.equal(T_1, T_b[b])
         assert torch.equal(idx_1, idx_b[b, : sizes_s[b]][idx_b[b, : sizes_s[b]] >= 0])
